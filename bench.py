@@ -3,6 +3,10 @@
 
   python bench.py --gpus N --steps K --warmup W          # this framework
   python bench.py --impl reference --gpus N ...          # CPU reference arm
+  python bench.py ... --dump-outputs DIR                 # + last-step outputs
+
+The inputs are generated from fixed seeds, so two builds run with the same
+arguments can be compared output for output through --dump-outputs.
 
 Prints ONE JSON line (rank 0).  The top-level keys are the contract line for
 BASELINE.json configs[1] (fused weighted RMSE + Bias + ACC, 6 variables x 13
@@ -64,6 +68,10 @@ RG_BYTES_PER_CELL = 4 + 4 * (RG_TLON * RG_TLAT) / (NLON * NLAT)
 SP_SLOTS = 37 * 5                     # (level, variable) outputs of the time mean
 SP_TIMES = 16                         # time steps per launch (12.3 GB)
 SP_NK = NLON // 2 + 1
+# --dump-outputs: outputs larger than this are sampled (same indices every run)
+DUMP_MAX_ELEMS = 1 << 20
+DUMP_SEED = 20240101
+DUMP_MAX_BYTES = 64 << 20
 
 
 def _peak_gbs():
@@ -455,6 +463,46 @@ class Harness:
     self.ctx.set_stream(self.stream.cuda_stream)
     self.sampler = ClockSampler(self.local)
     self.peak, self.peak_src = _peak_gbs()
+    self.outputs = {}  # name -> host array, for --dump-outputs
+
+  def keep(self, name, value):
+    """Records what a timed path returned in its last step for
+    --dump-outputs: a tensor, an array or an xarray_lite Dataset (one entry
+    per variable).  Outputs above DUMP_MAX_ELEMS elements are reduced to a
+    fixed, seeded sample of their flattened elements."""
+    if not self.args.dump_outputs:
+      return
+    if hasattr(value, 'keys'):
+      for v in value.keys():
+        self.keep(f'{name}.{v}', value[v].values)
+      return
+    torch = self.torch
+    if not isinstance(value, (np.ndarray, torch.Tensor)):
+      value = np.asarray(value.values)  # an xarray_lite DataArray
+    flat = value.reshape(-1)
+    if flat.shape[0] > DUMP_MAX_ELEMS:
+      rng = np.random.default_rng(DUMP_SEED)
+      idx = np.sort(rng.integers(0, flat.shape[0], DUMP_MAX_ELEMS))
+      if isinstance(flat, torch.Tensor):
+        idx = torch.from_numpy(idx).to(flat.device)
+      flat = flat[idx]
+      name += '.sample'
+    else:
+      flat = value
+    if isinstance(flat, torch.Tensor):
+      flat = flat.cpu().numpy()
+    flat = np.asarray(flat)
+    if flat.dtype not in (np.float32, np.float64):
+      flat = flat.astype(np.float64)
+    self.outputs[name] = np.array(flat)
+
+  def dump_outputs(self, out_dir):
+    """Writes the recorded outputs as <out_dir>/<name>.npy (rank 0)."""
+    total = sum(a.nbytes for a in self.outputs.values())
+    assert total <= DUMP_MAX_BYTES, total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in self.outputs.items():
+      np.save(os.path.join(out_dir, f'{name}.npy'), a)
 
   def barrier(self):
     if self.world > 1:
@@ -574,6 +622,7 @@ def bench_rmse_acc(h):
   # sanity (cheap, on rank 0): statistic 6 is the weight sum = nlat * nlon
   wsum = float(out[args.warmup, 0, 6].item())
   assert abs(wsum - SLAB) < 1e-3 * SLAB, wsum
+  h.keep('rmse_acc.stats', out[args.warmup + args.steps - 1])
   line = {
       'metric': 'grid-cells/s',
       'value': h.world * cells * args.steps / (ms_total * 1e-3),
@@ -657,6 +706,7 @@ def e2e_rmse_acc(h, f, t, c):
     ctx.reset_transfer_stats()
     dt, res, clocks = h.time_host(lambda i: chunk(1 + i), nsteps)
     st = ctx.transfer_stats()
+  h.keep('rmse_acc.e2e', res)
   d2h = sum(res[v].values.nbytes for v in res.keys())
   h.free_pinned(hf, ht, hc)
   return {'value': h.world * cells * nsteps / dt, 'unit': 'grid-cells/s',
@@ -713,6 +763,7 @@ def bench_crps(h):
   points = ENS_FIELDS * SLAB
   wsum = float(out[args.warmup, 0, 5].item())
   assert abs(wsum - SLAB) < 1e-3 * SLAB, wsum
+  h.keep('crps_sweep.stats', out[args.warmup + args.steps - 1])
   entry = {
       'workload': f'configs[2]: CRPS + spread/skill + ens-mean (R)MSE + variance, '
                   f'{ENS_M} members, {ENS_NVAR} vars x {NLEV} levels x '
@@ -769,6 +820,7 @@ def e2e_crps(h, x, t):
   ctx.reset_transfer_stats()
   dt, res, clocks = h.time_host(one, nsteps)
   st = ctx.transfer_stats()
+  h.keep('crps_sweep.e2e', res)
   d2h = sum(res[v].values.nbytes for v in res.keys())
   h.free_pinned(hx, ht)
   points = ENS_FIELDS * SLAB
@@ -807,6 +859,7 @@ def bench_regrid(h):
       step, lambda warm: None, args.steps, args.warmup)
   cells = RG_FIELDS * SLAB
   assert bool(torch.isfinite(out).all().item())
+  h.keep('regrid.out', out)
   entry = {
       'workload': f'configs[3]: ConservativeRegridder 0.25 -> 1.5 degree '
                   f'({NLAT}x{NLON} -> {RG_TLAT}x{RG_TLON}), 6 vars x 37 levels per '
@@ -831,6 +884,7 @@ def bench_regrid(h):
     dt, res, eclocks = h.time_host(lambda _: regridder.regrid_array(hx), nsteps)
     st = ctx.transfer_stats()
     assert res.shape == (RG_FIELDS, RG_TLON, RG_TLAT)
+    h.keep('regrid.e2e', res)
     h.free_pinned(hx)
     entry['e2e'] = {
         'value': h.world * cells * nsteps / dt, 'unit': 'source grid-cells/s',
@@ -874,6 +928,7 @@ def bench_spectrum(h):
                                                         args.warmup)
   cells = nfield * SLAB
   assert bool(torch.isfinite(acc).all().item())
+  h.keep('spectrum_sweep.time_sum', acc)
   entry = {
       'workload': f'configs[4]: zonal energy spectrum, rFFT along lon={NLON}, 37 '
                   f'levels x 5 vars, {SP_TIMES} time steps per launch '
@@ -899,6 +954,7 @@ def bench_spectrum(h):
 
   ms_total, ms_kernels, launches, rclocks = h.time_steps(
       step_red, tail_red, args.steps, args.warmup)
+  h.keep('spectrum_sweep.latsum', red)
   entry['latsum'] = {
       'what': 'north-star variant: rFFT + power + latitude-weighted meridional '
               'reduction (get_lat_weights) + time mean fused, nothing per-latitude '
@@ -926,6 +982,7 @@ def bench_spectrum(h):
         lambda _: op.compute(ds, time_sum_dim='time'), nsteps)
     st = ctx.transfer_stats()
     assert res.shape == (SP_SLOTS, NLAT, SP_NK)
+    h.keep('spectrum_sweep.e2e', res)
     h.free_pinned(hx)
     entry['e2e'] = {
         'value': h.world * cells * nsteps / dt, 'unit': 'grid-cells/s',
@@ -951,6 +1008,11 @@ def main():
   ap.add_argument('--workloads', default='crps,regrid,spectrum',
                   help='comma-separated subset of crps,regrid,spectrum (the '
                        'configs[1] line always runs); "none" skips them')
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='after the timed steps, write what each timed path '
+                       'returned in its last step as DIR/<name>.npy (rank 0; '
+                       'outputs above 2**20 elements as a fixed, seeded '
+                       'sample; at most 64 MB in all)')
   args = ap.parse_args()
   if args.impl == 'reference':
     run_reference(args)
@@ -985,6 +1047,8 @@ def main():
         workloads[name]['cpu_baseline'] = cpu_baseline_single(key, reps=2)
     line['cpu_baseline']['host'] = usable_cores()[1]
   if h.rank == 0:
+    if args.dump_outputs:
+      h.dump_outputs(args.dump_outputs)
     print(json.dumps(line))
   if h.world > 1:
     h.dist.destroy_process_group()

@@ -15,6 +15,7 @@ from __future__ import annotations
 
 import contextlib
 import ctypes as C
+import hashlib
 
 import numpy as np
 
@@ -45,6 +46,7 @@ class FakeContext:
     self._bufs: dict = {}
     self.calls: list = []
     self.h2d_bytes = 0
+    self._cached = None  # host address -> digest of the slab, in slab_cache()
 
   # -- memory -------------------------------------------------------------------
   def malloc(self, nbytes: int) -> int:
@@ -87,8 +89,33 @@ class FakeContext:
         n += 1
     return n
 
+  @contextlib.contextmanager
   def slab_cache(self, nbytes=None):
-    return contextlib.nullcontext()
+    """Holds the library's slab-cache contract: the truth / climatology slabs
+    a *_host entry reads are keyed by host address, so an address that comes
+    back with other contents inside the scope (a freed per-chunk copy
+    reallocated in place) would be served stale by the library.  Re-entrant,
+    like Context.slab_cache."""
+    del nbytes
+    if self._cached is not None:
+      yield self
+      return
+    self._cached = {}
+    try:
+      yield self
+    finally:
+      self._cached = None
+
+  def _check_cached(self, base, offs, w, dtype):
+    if self._cached is None:
+      return
+    es = np.dtype(dtype).itemsize
+    for off in offs:
+      addr = base + int(off) * es
+      digest = hashlib.blake2b(
+          _slab(base, off, w, dtype, native=True).tobytes()).digest()
+      assert self._cached.setdefault(addr, digest) == digest, (
+          f'slab cache: host address {addr:#x} reused with other contents')
 
   def pinned_result(self, shape, dtype):
     return np.empty(shape, dtype=dtype)
@@ -124,6 +151,10 @@ class FakeContext:
                   out, host=False):
     self.calls.append(('det_metrics', int(off_f.size), weights.nregion, host))
     dt = np.float32 if dtype == _lib.F32 else np.float64
+    if host:
+      self._check_cached(t, off_t, weights, dt)
+      if c:
+        self._check_cached(c, off_c, weights, dt)
     W = self._weights(weights)
     res = np.zeros((off_f.size, weights.nregion, _lib.DET_NSTAT))
     for i in range(off_f.size):
@@ -201,6 +232,7 @@ class FakeContext:
 
   def ens_metrics_host(self, x, t, nmember, member_stride, off_x, off_t,
                        weights, skipna, out):
+    self._check_cached(t, off_t, weights, np.float32)
     self.ens_metrics(x, t, _lib.F32, nmember, member_stride, off_x, off_t,
                      weights, skipna, out)
 
@@ -582,13 +614,25 @@ def _quiet():
     yield
 
 
+_installed = 0  # depth of the installed() blocks being executed
+
+
+def active() -> bool:
+  """Whether the stand-in is installed: test bodies shared with the GPU suite
+  then keep to host inputs, even on a machine that has a GPU."""
+  return _installed > 0
+
+
 @contextlib.contextmanager
 def installed():
   """Makes `_lib.default_context()` return a FakeContext inside the block."""
+  global _installed
   fake = FakeContext()
   saved = _lib.default_context
   _lib.default_context = lambda device=None: fake
+  _installed += 1
   try:
     yield fake
   finally:
+    _installed -= 1
     _lib.default_context = saved

@@ -161,10 +161,22 @@ def _truth_for_chunk(truth, fc, chunk_dim, select_truth):
   aligned BY LABEL like the reference's xarray arithmetic -- the truth record
   may be longer than the forecast's or start elsewhere -- never by position;
   forecast times without a truth label raise KeyError (an inner join would
-  silently shorten the time mean)."""
+  silently shorten the time mean).
+
+  The by-valid truth is a lazily gathered view of the truth record, not a
+  per-chunk copy: the slab cache keys truth slabs by host address, and a copy
+  freed after one chunk can be reallocated at the same address for the next
+  one with other contents."""
   tr = select_truth(truth, fc)
   if chunk_dim == 'time' and 'time' in truth.dims and 'time' in fc.coords:
-    tr = truth.sel(time=fc.coords['time'].values)
+    times = fc.coords['time'].values
+    pos = xl._lookup(truth.coords['time'].values, times)  # pylint: disable=protected-access
+    tr = xl.Dataset(attrs=truth.attrs)
+    for k in truth.keys():
+      v = truth[k]
+      tr[k] = v if 'time' not in v.dims else xl.LazyGather(
+          v, {'time': (('time',), pos)},
+          extra_coords={'time': xl.Coord(('time',), times)})
   return tr
 
 
